@@ -2,7 +2,7 @@
 """bench.py -- images/sec of the C2 hot path: 1080p JPEG decode -> Resize(224x224) -> CropMirrorNormalize fp16 CHW,
 batch 256 per GPU (BASELINE.json metric, configs[1]), weak scaling over N GPUs of one node.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   (N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...)
 
 One JSON line on rank 0.  `value` = device-resident throughput (encoded bytes already in HBM when the timed
@@ -249,6 +249,13 @@ class CpuReference:
             self.pool = None
 
 
+def dump_sample(batch):
+    """Indices of the images `--dump-outputs` keeps: the whole [batch, 3, 224, 224] output as float32 is 154 MB at batch 256,
+    so a fixed, seeded sample of whole images is kept (60 MiB: under 64 MB with the index and the .npy headers), sorted."""
+    n = min(batch, (60 << 20) // (3 * OUT * OUT * 4))
+    return np.sort(np.random.default_rng(0).choice(batch, n, replace=False))
+
+
 def reference_arm(batch, cores, steps, warmup, dump=None):
     """Times the reference CPU path (bounded sample per step) and returns the JSON fields shared by `--impl reference` and
     the `cpu_baseline` leg of our arm."""
@@ -257,7 +264,7 @@ def reference_arm(batch, cores, steps, warmup, dump=None):
     mirror = np.random.default_rng(0).integers(0, 2, sample)
     ref = CpuReference(streams, cores)
     try:
-        for _ in range(max(1, min(warmup, 2))):
+        for _ in range(warmup):
             ref.run(min(sample, max(2, cores)), mirror)
         times = []
         for _ in range(steps):
@@ -383,13 +390,21 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=10)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--warmup", type=int, default=3, help="untimed steps in front of every timed leg")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=BATCH)
     ap.add_argument("--no-secondary", action="store_true", help="skip the C3 (video) and C4 (audio) secondary measurements")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU baseline leg of our arm")
     ap.add_argument("--dump", default=None, help="(reference arm) save the outputs of the sample as .npy")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed to DIR/*.npy (float32; a fixed, seeded "
+                         "sample of the images when the whole batch exceeds 64 MB); --impl ours only: the reference arm "
+                         "computes a bounded CPU sample of other size, which --dump saves")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -420,7 +435,7 @@ def main():
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         import tempfile
         cpu_dump = os.path.join(tempfile.gettempdir(), f"dalib200_cpu_ref_{os.getpid()}.npy")
-        cpu_baseline, cpu_sample = reference_arm(batch, cores, 2, 1, dump=cpu_dump)
+        cpu_baseline, cpu_sample = reference_arm(batch, cores, args.steps, args.warmup, dump=cpu_dump)
 
     # ------------------------------------------------------------------ our arm
     import torch
@@ -467,7 +482,6 @@ def main():
     for _ in range(args.warmup):
         pipe.launch()
     torch.cuda.synchronize()
-    assert all(s == 0 for s in pipe.status()), "decoder reported a truncated stream"
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
     capi.profiling(True)
     capi.profiling_collect()
@@ -488,6 +502,14 @@ def main():
     prof = capi.profiling_collect()
     capi.profiling(False)
     step_ms = [a.elapsed_time(b) for a, b in ev]
+    # read after the timed steps: the decoder has no status before its first launch (--warmup 0)
+    assert all(s == 0 for s in pipe.status()), "decoder reported a truncated stream"
+    # the output of the last timed step, read before anything launches the pipeline again
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        keep = dump_sample(batch)
+        dumped = {"c2_output": pipe.output[torch.from_numpy(keep).cuda()].float().cpu().numpy(),
+                  "c2_output_sample_index": keep.astype(np.float64)}
     total_ms = float(sum(step_ms))
     if world > 1:
         t = torch.tensor([total_ms], device="cuda", dtype=torch.float64)
@@ -554,7 +576,7 @@ def main():
         (out,) = api_pipe.run()
         t = torch.as_tensor(out.as_tensor(), device="cuda")
         return t, float(t[:, 0, 0, 0].float().sum().item())      # D2H read of a result scalar
-    for _ in range(max(1, min(args.warmup, 2))):
+    for _ in range(args.warmup):
         api_out, chk = e2e_step()
     barrier()
     t0 = time.perf_counter()
@@ -588,7 +610,7 @@ def main():
     if rank == 0 and world == 1 and not args.no_secondary:
         del api_pipe
         try:
-            secondary = secondary_workloads(hbm_peak, flush, max(3, args.steps // 2), 2)
+            secondary = secondary_workloads(hbm_peak, flush, args.steps, args.warmup)
         except Exception as ex:           # the headline line must not depend on the secondary workloads
             secondary = {"error": repr(ex)}
     # ---- optional consumer-side collective (BASELINE configs[4]): all-gather of the fp16 NCHW output of every rank over NVLink.
@@ -628,6 +650,10 @@ def main():
                 "kernels": kernels, "op_boundary_GBps": op_gbs, "op_boundary_frac_of_hbm": op_gbs / hbm_peak,
                 "wall_s_timed_region": t_wall, "checksum": chk, "secondary": secondary, "allgather_fp16_nchw": allgather}
         print(json.dumps(line))
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     if world > 1:
         dist.destroy_process_group()
     return 0
