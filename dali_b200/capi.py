@@ -41,6 +41,8 @@ EXPORTS = [
     "dalib200GenericPlanCreate", "dalib200GenericPlanDestroy", "dalib200MultiplyAddSetup", "dalib200WindowCopySetup", "dalib200GenericLaunch",
     "dalib200MelPlanCreate", "dalib200MelPlanDestroy", "dalib200MelPlanSetup", "dalib200MelLaunch", "dalib200MelPlanSetTensorCores",
     "dalib200SpectrogramMelSupported", "dalib200SpectrogramMelLaunch",
+    "dalib200SepConvPlanCreate", "dalib200SepConvPlanDestroy", "dalib200SepConvPlanSetup", "dalib200SepConvLaunch",
+    "dalib200SepConvPlanGetPath", "dalib200GaussianWindow",
 ]
 
 
@@ -76,6 +78,11 @@ class Resample3DSample(C.Structure):
     _fields_ = [("in_shape", C.c_int32 * 3), ("channels", C.c_int32), ("out_shape", C.c_int32 * 3),
                 ("use_roi", C.c_int32 * 3), ("roi_start", C.c_float * 3), ("roi_end", C.c_float * 3),
                 ("min_filter", FilterDesc * 3), ("mag_filter", FilterDesc * 3)]
+
+
+class SepConvSample(C.Structure):
+    _fields_ = [("ndim", C.c_int32), ("shape", C.c_int32 * 3), ("channels", C.c_int32), ("diameter", C.c_int32 * 3),
+                ("window_offset", C.c_int32 * 3)]
 
 
 class CmnSample(C.Structure):
@@ -133,6 +140,9 @@ def lib():
         _lib.dalib200GetLaunchCount.restype = C.c_uint64
         _lib.dalib200JpegPlanStagedBytes.restype = C.c_size_t
         _lib.dalib200SpectrogramNumWindows.restype = C.c_int64
+        _lib.dalib200GaussianWindow.restype = None
+        _lib.dalib200GaussianWindow.argtypes = [C.c_float, C.c_int, C.c_void_p]
+        _lib.dalib200SepConvPlanSetup.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int]
     return _lib
 
 

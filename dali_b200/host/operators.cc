@@ -2348,6 +2348,150 @@ class NormalizeGPU : public SignalOpBase {
 };
 DALI_REGISTER_OPERATOR(Normalize, NormalizeGPU, GPU);
 
+// =============================================================================================== GaussianBlur
+// dali/operators/image/convolution/gaussian_blur.cc (schema), gaussian_blur_params.h (per-axis sigma / window resolution),
+// gaussian_blur_gpu.cu; the convolution itself is dalib200SepConv* (separable, reflect-101, innermost axis first).
+DALI_SCHEMA(GaussianBlur)
+    .DocStr("Applies a Gaussian Blur to the input.\n\nGaussian blur is calculated by applying a convolution with a Gaussian kernel, "
+            "which can be parametrized with `windows_size` and `sigma`. If only the sigma is specified, the radius of the kernel "
+            "is 3 * sigma (rounded up), so the kernel window size is 2 * ceil(3 * sigma) + 1. If only the window size is provided, "
+            "the sigma is calculated by using the following formula: radius = (window_size - 1) / 2; "
+            "sigma = (radius - 1) * 0.3 + 0.8. The sigma and kernel window size can be specified as one value for all data "
+            "axes or a value per data axis. When specifying the sigma or window size per axis, the axes are provided same as "
+            "layouts, from outermost to innermost. The channel C dimension and the frame F dimension are not blurred.")
+    .NumInput(1).NumOutput(1).AllowSequences()
+    .AddOptionalArg("window_size", "The diameter of the kernel.", std::vector<int>{0}, true)
+    .AddOptionalArg("sigma", "Sigma value for the Gaussian Kernel.", std::vector<float>{0.0f}, true)
+    .AddOptionalArgNoDefault("dtype", "Output data type.\n\nSupported type: `FLOAT`. If not set, the input type is used.");
+
+namespace gaussian_detail {
+// channel-last layouts with an optional leading F; returns false for anything else
+inline bool ParseLayout(const std::string &l, bool *frames, int *spatial) {
+  static const char *const kLayouts[] = { "HW", "HWC", "FHW", "FHWC", "DHW", "DHWC", "FDHW", "FDHWC" };
+  bool known = false;
+  for (const char *k : kLayouts) known |= l == k;
+  if (!known) return false;
+  *frames = l[0] == 'F';
+  *spatial = l.find('D') == std::string::npos ? 2 : 3;
+  return true;
+}
+// GaussianBlurParams (gaussian_blur_params.h): window_size = 2 * ceil(3 sigma) + 1 when only sigma is given,
+// sigma = (radius - 1) * 0.3 + 0.8 when only the window is given
+inline void ResolveAxis(float sigma, float window, int sample, int axis, float *sigma_out, int *diameter_out) {
+  DALI_ENFORCE(window == std::floor(window) && window >= 0 && window <= 1e9f, "GaussianBlur: sample ", sample, " axis ", axis,
+               ": `window_size` must be a non-negative integer, got ", window);
+  const int ws = static_cast<int>(window);
+  DALI_ENFORCE(ws == 0 || ws % 2 == 1, "GaussianBlur: sample ", sample, " axis ", axis, ": kernel window should have odd length, got: ", ws);
+  DALI_ENFORCE(sigma >= 0, "GaussianBlur: sample ", sample, " axis ", axis, ": sigma must be non-negative, got: ", sigma);
+  DALI_ENFORCE(!(sigma == 0 && ws == 0), "GaussianBlur: sample ", sample, " axis ", axis,
+               ": `sigma` and `window_size` shouldn't be 0 at the same time");
+  int d = ws;
+  if (d == 0) {
+    const float r = std::ceil(sigma * 3);
+    DALI_ENFORCE(r <= 1e6f, "GaussianBlur: sample ", sample, " axis ", axis, ": sigma ", sigma, " is too large");
+    d = 2 * static_cast<int>(r) + 1;
+  }
+  float s = sigma;
+  if (s == 0) s = static_cast<float>(((d - 1) / 2 - 1) * 0.3 + 0.8);
+  *sigma_out = s;
+  *diameter_out = d;
+}
+}  // namespace gaussian_detail
+
+class GaussianBlurGPU : public Operator<GPUBackend> {
+ public:
+  explicit GaussianBlurGPU(const OpSpec &spec) : Operator<GPUBackend>(spec) {
+    CheckStatus(dalib200SepConvPlanCreate(&plan_, max_batch_size_ * 64), "GaussianBlur");
+    plan_cap_ = max_batch_size_ * 64;
+  }
+  ~GaussianBlurGPU() override { dalib200SepConvPlanDestroy(plan_); }
+ protected:
+  bool SetupImpl(std::vector<OutputDesc> &out, const Workspace &ws) override {
+    const auto &in = ws.Input<GPUBackend>(0);
+    DALI_ENFORCE(in.type() == DALI_UINT8 || in.type() == DALI_FLOAT,
+                 "GaussianBlur: the GPU path supports uint8 and float inputs, got type ", static_cast<int>(in.type()));
+    out_type_ = spec_.ArgumentDefined("dtype") ? spec_.GetArgument<DALIDataType>("dtype") : in.type();
+    DALI_ENFORCE(out_type_ == in.type() || out_type_ == DALI_FLOAT, "GaussianBlur: output type must be the input type or FLOAT");
+    const int nd = in.shape().sample_dim();
+    layout_ = in.GetLayout().str();
+    if (layout_.empty()) layout_ = nd == 3 ? "HWC" : nd == 4 ? "FHWC" : "";
+    bool frames = false;
+    int spatial = 2;
+    DALI_ENFORCE(gaussian_detail::ParseLayout(layout_, &frames, &spatial), "GaussianBlur: unsupported layout \"", layout_,
+                 "\" (", nd, "-D input); expected one of HW, HWC, FHW, FHWC, DHW, DHWC, FDHW, FDHWC");
+    DALI_ENFORCE(static_cast<int>(layout_.size()) == nd, "GaussianBlur: layout \"", layout_, "\" does not match a ", nd, "-D input");
+    const bool has_c = layout_.back() == 'C';
+    const int fs = frames ? 1 : 0;
+    const int n = in.num_samples();
+    samples_.clear();
+    frame_sample_.clear();
+    frame_off_.clear();
+    std::vector<float> windows;
+    std::map<std::pair<uint32_t, int>, int32_t> seen;      // (sigma bits, diameter) -> offset: one window per distinct pair
+    for (int i = 0; i < n; i++) {
+      const int64_t *s = in.shape().tensor_shape_span(i);
+      const auto sig = spec_.GetFloatVecArgument("sigma", &ws, i, spatial);
+      const auto win = spec_.GetFloatVecArgument("window_size", &ws, i, spatial);
+      dalib200SepConvSample cs{};
+      cs.ndim = spatial;
+      cs.channels = has_c ? static_cast<int32_t>(s[nd - 1]) : 1;
+      for (int a = 0; a < spatial; a++) {
+        DALI_ENFORCE(s[fs + a] < (int64_t{1} << 31), "GaussianBlur: extent too large");
+        cs.shape[a] = static_cast<int32_t>(s[fs + a]);
+        float sigma;
+        int d;
+        gaussian_detail::ResolveAxis(sig[a], win[a], i, a, &sigma, &d);
+        DALI_ENFORCE(d <= 8191, "GaussianBlur: sample ", i, " axis ", a, ": window of ", d, " taps exceeds the limit of 8191");
+        uint32_t bits;
+        std::memcpy(&bits, &sigma, 4);
+        auto it = seen.find({bits, d});
+        if (it == seen.end()) {
+          it = seen.emplace(std::make_pair(bits, d), static_cast<int32_t>(windows.size())).first;
+          windows.resize(windows.size() + d);
+          dalib200GaussianWindow(sigma, d, windows.data() + it->second);
+        }
+        cs.diameter[a] = d;
+        cs.window_offset[a] = it->second;
+      }
+      const int64_t nframes = frames ? s[0] : 1;
+      int64_t fe = cs.channels;
+      for (int a = 0; a < spatial; a++) fe *= cs.shape[a];
+      for (int64_t k = 0; k < nframes; k++) { samples_.push_back(cs); frame_sample_.push_back(i); frame_off_.push_back(k * fe); }
+    }
+    const int nf = static_cast<int>(samples_.size());
+    if (nf > plan_cap_) { dalib200SepConvPlanDestroy(plan_); plan_ = nullptr; plan_cap_ = nf; CheckStatus(dalib200SepConvPlanCreate(&plan_, nf), "GaussianBlur"); }
+    CheckStatus(dalib200SepConvPlanSetup(plan_, nf, samples_.data(), windows.data(), static_cast<int64_t>(windows.size()),
+                                         in.type() == DALI_UINT8 ? DALIB200_UINT8 : DALIB200_FLOAT,
+                                         out_type_ == DALI_UINT8 ? DALIB200_UINT8 : DALIB200_FLOAT), "GaussianBlur");
+    out.resize(1);
+    out[0].shape = in.shape(); out[0].type = out_type_;
+    return true;
+  }
+  void RunImpl(Workspace &ws) override {
+    const auto &in = ws.Input<GPUBackend>(0);
+    auto &out = ws.Output<GPUBackend>(0);
+    out.SetLayout(TensorLayout(layout_));
+    const int nf = static_cast<int>(samples_.size());
+    std::vector<const void *> ip(nf);
+    std::vector<void *> op(nf);
+    const size_t ies = TypeSize(in.type()), oes = TypeSize(out_type_);
+    for (int k = 0; k < nf; k++) {
+      ip[k] = static_cast<const uint8_t *>(in.raw_tensor(frame_sample_[k])) + frame_off_[k] * ies;
+      op[k] = static_cast<uint8_t *>(out.raw_mutable_tensor(frame_sample_[k])) + frame_off_[k] * oes;
+    }
+    CheckStatus(dalib200SepConvLaunch(plan_, ip.data(), op.data(), ws.stream()), "GaussianBlur");
+  }
+ private:
+  dalib200SepConvPlan *plan_ = nullptr;
+  int plan_cap_ = 0;
+  DALIDataType out_type_ = DALI_UINT8;
+  std::string layout_;
+  std::vector<dalib200SepConvSample> samples_;
+  std::vector<int> frame_sample_;        // frame -> sample
+  std::vector<int64_t> frame_off_;       // element offset of the frame inside its sample
+};
+DALI_REGISTER_OPERATOR(GaussianBlur, GaussianBlurGPU, GPU);
+
 }  // namespace dali
 
 // ---------------------------------------------------------------------------------------------------------------

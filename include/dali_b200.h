@@ -398,6 +398,38 @@ int dalib200MultiplyAddSetup(dalib200GenericPlan *plan, int n, const int64_t *vo
 int dalib200WindowCopySetup(dalib200GenericPlan *plan, int n, const dalib200WindowSample *samples);
 int dalib200GenericLaunch(dalib200GenericPlan *plan, const void *const *in_ptrs, void *const *out_ptrs, dalib200Stream_t stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Separable convolution with reflect-101 borders (fn.gaussian_blur).  Replaces kernels::SeparableConvolutionGpu
+ * (dali/kernels/imgproc/convolution/separable_convolution_gpu.h) behind GaussianBlurOpGpu
+ * (dali/operators/image/convolution/gaussian_blur_gpu.cu); numerics follow SeparableConvolutionCpu
+ * (separable_convolution_cpu.h, convolution_cpu.h) -- the parity target: passes innermost axis first, fp32 intermediates,
+ * taps summed in ascending order with separately rounded products and sums.
+ * A sample is one channel-last 2-D frame (HW / HWC) or volume (DHW / DHWC); the caller flattens sequences into frames. */
+typedef struct dalib200SepConvPlan dalib200SepConvPlan;
+
+typedef struct {
+  int32_t ndim;               /* spatial rank: 2 or 3 */
+  int32_t shape[3];           /* spatial extents, outermost first: (H, W) or (D, H, W) */
+  int32_t channels;
+  int32_t diameter[3];        /* window length per axis, same order; odd, 1 .. 8191 */
+  int32_t window_offset[3];   /* first tap of each axis' window in the caller's window array */
+} dalib200SepConvSample;
+
+int dalib200SepConvPlanCreate(dalib200SepConvPlan **plan, int max_batch);
+int dalib200SepConvPlanDestroy(dalib200SepConvPlan *plan);
+/* windows: host array of num_window_floats taps that the samples index into (windows shared by several samples are stored once
+ * in the plan's coefficient table).  in_dtype / out_dtype: u8 -> u8, u8 -> f32, f32 -> f32. */
+int dalib200SepConvPlanSetup(dalib200SepConvPlan *plan, int n, const dalib200SepConvSample *samples, const float *windows,
+                             int64_t num_window_floats, int in_dtype, int out_dtype);
+/* in_ptrs[i] / out_ptrs[i]: device buffers of the sample's shape x channels (output shape = input shape) */
+int dalib200SepConvLaunch(dalib200SepConvPlan *plan, const void *const *in_ptrs, void *const *out_ptrs, dalib200Stream_t stream);
+/* introspection used by the tests: 1 = streaming 2-D kernel (TMA row ring), 0 = per-axis pass kernels, -1 = bad index.  The path of
+ * the last launch (before the first launch: the setup's choice, which a launch demotes to 0 for an input not 16-byte aligned). */
+int dalib200SepConvPlanGetPath(const dalib200SepConvPlan *plan, int sample);
+/* host helper: FillGaussian (dali/operators/image/convolution/gaussian_blur_params.h) -- `diameter` taps of the normalised Gaussian
+ * of `sigma`, computed in double and rounded to float per tap */
+void dalib200GaussianWindow(float sigma, int diameter, float *out);
+
 #ifdef __cplusplus
 }
 #endif

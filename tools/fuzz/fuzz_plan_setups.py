@@ -61,7 +61,7 @@ def note(name, rc):
     hist[(name, "ok" if rc == 0 else "err")] = hist.get((name, "ok" if rc == 0 else "err"), 0) + 1
 
 
-plans = {k: plan(k, 8) for k in ("Resample", "Resample3D", "Cmn", "Warp", "Pointwise", "Spectrogram", "Mel", "Signal", "Generic")}
+plans = {k: plan(k, 8) for k in ("Resample", "Resample3D", "Cmn", "Warp", "Pointwise", "Spectrogram", "Mel", "Signal", "Generic", "SepConv")}
 for it in range(N):
     n = int(rng.integers(0, 9)) if rng.random() < 0.9 else int(rng.choice([9, 100, -1]))
     m = max(n, 1) if n < 64 else 8
@@ -233,4 +233,23 @@ for it in range(N):
     note("window_copy", rc)
     if rc == 0:
         launch("window_copy", L.dalib200GenericLaunch, plans["Generic"].handle, fake_ptrs(m, 0x10000000), fake_ptrs(m, 0x7000000000), None)
+    # ---- separable convolution: zero / negative / 2^31 extents, even / zero / huge diameters, windows outside the array, NaN / inf taps
+    nw = int(rng.choice([0, 1, 7, 64, 300]))
+    wins = np.ascontiguousarray(rng.uniform(0, 1, max(nw, 1)), np.float32)
+    if nw and rng.random() < 0.1 * MILD:
+        wins[int(rng.integers(0, nw))] = float(rng.choice([float("nan"), float("inf"), float("-inf")]))
+    SC = (capi.SepConvSample * m)()
+    for s in SC:
+        s.ndim, s.channels = code([2, 3]), small(1, 5)
+        for a in range(3):
+            s.shape[a] = dim(0, 300)
+            s.diameter[a] = int(rng.choice(BAD_I)) if rng.random() < 0.1 * MILD else 2 * int(rng.integers(0, 12)) + 1
+            s.window_offset[a] = int(rng.choice(BAD_I)) if rng.random() < 0.05 * MILD else int(rng.integers(0, max(nw - s.diameter[a], 0) + 1))
+    rc = L.dalib200SepConvPlanSetup(plans["SepConv"].handle, n, SC, wins.ctypes.data, nw, code([0, 9]), code([0, 9]))
+    note("sepconv", rc)
+    # the launch allocates the float temporaries for real (calloc in the stub): only batches of a plausible size are launched
+    if rc == 0 and sum(int(np.prod([s.shape[a] for a in range(s.ndim)], dtype=np.int64)) * s.channels for s in SC[:max(n, 0)]) < 2 ** 27:
+        launch("sepconv", L.dalib200SepConvLaunch, plans["SepConv"].handle, fake_ptrs(m, 0x10000000), fake_ptrs(m, 0x7000000000), None)
+        for i in range(max(0, min(n, m))):
+            L.dalib200SepConvPlanGetPath(plans["SepConv"].handle, i)
 print("seed", sys.argv[1] if len(sys.argv) > 1 else 0, "iterations", N, "- no sanitizer report;", {f"{k[0]}:{k[1]}": v for k, v in sorted(hist.items())})
